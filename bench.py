@@ -14,7 +14,13 @@ N > 1 : one step = fusedL2NN 1,000,000 queries x 8,000,000 db rows x 96 (configs
         against the exact fp64 arg-min over its own shard (combined across ranks) -> "parity".
 --impl reference : the CPU restatement (oracle port: numpy expanded form on multithreaded BLAS,
         all host cores) on a bounded sample of the same workload.  The reference's own kernels for
-        this path are not in /root/reference (SURVEY.md section 0), so there is nothing else to run.
+        this path are not in the reference snapshot (SURVEY.md section 0), so there is nothing else to run.
+--dump-outputs DIR : after the timed steps, what the last timed step returned is written as DIR/<name>.npy
+        (float32 / float64, 32 MB at N = 1, 12 MB at N > 1), so that two builds run with the same arguments
+        (same seeded inputs) can be compared output for output:
+          N = 1 : pairwise_distance.npy -- the [2048, 4096] float32 sub-matrix of the 100000 x 100000 result at
+                  rows / columns drawn by torch.randperm with seed 5 (sorted), see DUMP_SAMPLE
+          N > 1 : fused_l2_nn_idx.npy (float64, exact) and fused_l2_nn_val.npy (float32), all 1M queries (rank 0)
 """
 from __future__ import annotations
 
@@ -33,6 +39,7 @@ sys.path.insert(0, ROOT)
 PAIRWISE = dict(m=100_000, n=100_000, k=128)
 FUSED_NN = dict(m=1_000_000, n=8_000_000, k=96)
 METRIC = "distance-pairs/sec"
+DUMP_SAMPLE = dict(rows=2048, cols=4096, seed=5)   # --dump-outputs at N = 1: the full result is 40 GB
 
 
 def measured_peaks():
@@ -214,6 +221,24 @@ def time_steps(fn, steps, warmup, torch, sync_all=None):
     return total / steps, per
 
 
+def dump_outputs(dirname, arrays):
+    """--dump-outputs: {name: tensor} -> dirname/<name>.npy; integer outputs as float64 (exact below 2^53)."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        a = a.astype(np.float64 if a.dtype.kind in "iu" or a.dtype == np.float64 else np.float32)
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
+def pairwise_dump_sample(out, torch):
+    """The fixed DUMP_SAMPLE sub-matrix of a pairwise result (sorted seeded rows x sorted seeded columns)."""
+    g = torch.Generator(device=out.device).manual_seed(DUMP_SAMPLE["seed"])
+    rows = torch.randperm(out.shape[0], device=out.device, generator=g)[:DUMP_SAMPLE["rows"]].sort().values
+    cols = torch.randperm(out.shape[1], device=out.device, generator=g)[:DUMP_SAMPLE["cols"]].sort().values
+    return out[rows[:, None], cols[None, :]]
+
+
 def gpu_baselines_pairwise(x, y, out, m, n, k, ours_ms, torch, steps=5, warm=2):
     """GPU baselines for configs[1] (L2Expanded m x n x k fp32), timed like the engine (CUDA events, output buffer
     reused; every step streams 40+ GB through the 126 MB L2, so nothing is cached between steps)."""
@@ -340,6 +365,8 @@ def run_pairwise_1gpu(args):
     k_ms = sum(kernel_ms) / len(kernel_ms) if kernel_ms else ms
     clocks = cs.summary()
     pairs = m * n
+    if args.dump_outputs:            # before the other configs below reuse `out`
+        dump_outputs(args.dump_outputs, {"pairwise_distance": pairwise_dump_sample(out, torch)})
     # ---- parity of what was just timed: the result of the last timed step, re-evaluated in fp64 on the device
     parity = dc.check_pairwise_sampled(out, x, y, 0, count=200_000, eps=1e-4)
     parity["what"] = "L2Expanded 100000x100000x128: sampled pairs incl. tile corners / matrix edges vs fp64, CompareApprox(1e-4)"
@@ -539,6 +566,8 @@ def run_fused_nn_multi(args):
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms = float(t.item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"fused_l2_nn_idx": last["iv"][0], "fused_l2_nn_val": last["iv"][1]})
     # ---- parity on EVERY rank: the reduced result vs the exact fp64 arg-min (own shard, combined across ranks)
     g = torch.Generator(device=dev).manual_seed(3)
     rows = torch.randperm(m, device=dev, generator=g)[:8192]
@@ -648,7 +677,13 @@ def main():
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return run_reference(args)

@@ -15,4 +15,10 @@ def pytest_configure(config):
 @pytest.fixture(scope="session")
 def golden():
     import numpy as np
-    return np.load(os.path.join(ROOT, "tests", "golden", "distance_golden.npz"))
+    with np.load(os.path.join(ROOT, "tests", "golden", "distance_golden.npz")) as z:
+        g = dict(z)
+    # the unexpanded L2 forms are the same cdist values as the expanded ones, stored once (make_golden.py)
+    for case in ("small", "cfg1"):
+        g[f"{case}_L2Unexpanded"] = g[f"{case}_L2Expanded"]
+        g[f"{case}_L2SqrtUnexpanded"] = g[f"{case}_L2SqrtExpanded"]
+    return g

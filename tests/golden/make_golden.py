@@ -15,8 +15,9 @@ from scipy.spatial.distance import cdist
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 SCIPY = {"L2Expanded": "sqeuclidean", "L2SqrtExpanded": "euclidean", "CosineExpanded": "cosine",
-         "L1": "cityblock", "L2Unexpanded": "sqeuclidean", "L2SqrtUnexpanded": "euclidean",
-         "Linf": "chebyshev", "Canberra": "canberra", "CorrelationExpanded": "correlation"}
+         "L1": "cityblock", "Linf": "chebyshev", "Canberra": "canberra", "CorrelationExpanded": "correlation"}
+# L2Unexpanded / L2SqrtUnexpanded have the same exact values as the expanded forms: stored once, aliased by the
+# `golden` fixture in tests/conftest.py (keeps the file under 1 MB)
 
 
 def blobs(rows, cols, seed, centers=None):
